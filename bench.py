@@ -1,6 +1,6 @@
 """bench.py -- end-to-end tracked frames/s (detect + NMS + associate) of the B200-native path, and the CPU reference arm.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload pipeline|tracker]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload pipeline|tracker] [--dump-outputs DIR]
 
 Default workload "pipeline" (bench_pipeline.py) = the BASELINE.json metric: YOLOv7-w6 1280 x 1280, batch 8 -> decode + NMS ->
 ByteTrack, one uint8 frame per sequence per step; its JSON line also carries BASELINE configs C1 / C3 / C4 / C5, C4 end to end with the
@@ -180,7 +180,7 @@ def run_reference_arm(args, rank, world):
 def parse_args():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=None, help="timed steps (default: 200 pipeline, 1500 tracker-only)")
+    ap.add_argument("--steps", type=int, default=None, help="timed steps (default: 100 pipeline, 1500 tracker-only; 20 and 200 with --impl reference)")
     ap.add_argument("--warmup", type=int, default=20)
     ap.add_argument("--impl", default="ours")
     ap.add_argument("--seqs", type=int, default=4)
@@ -194,7 +194,41 @@ def parse_args():
     ap.add_argument("--no-sub", action="store_true", help="pipeline: skip config.sub_benchmarks (C3 / C4 / C5)")
     ap.add_argument("--quick-sub", action="store_true", help="pipeline: shorter sub-benchmarks")
     ap.add_argument("--no-cpu", action="store_true", help="pipeline: skip the cpu_baseline leg")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step returned as DIR/<name>.npy (float64)")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
+    return args
+
+
+def track_outputs(rows, stat):
+    """What a tracker step returns, for dump_outputs: the track rows, with the rows past each sequence's count (stale buffer
+    contents) zeroed, and the result counters (the stat words from STAT_PHASE0 on are clock-cycle counts, not results)."""
+    from b200track import _lib as L
+    rows, stat = np.array(rows, dtype=np.float64), np.asarray(stat)
+    for s, n in enumerate(stat[:, L.STAT_NOUT]):
+        rows[s, int(n):] = 0
+    return {"tracks": rows, "stat": stat[:, :L.STAT_PHASE0]}
+
+
+DUMP_BYTES = 64 * 10 ** 6
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes every array as out_dir/<name>.npy in float64: the inputs are seeded, so two builds run with the same arguments
+    can be compared output for output.  The leading axis of every array is the sequence; when all of them would take more than
+    DUMP_BYTES, the same fixed, seeded sample of sequences is written from each, and its indices as sequence_index.npy."""
+    arrays = {name: np.asarray(a, dtype=np.float64) for name, a in arrays.items()}
+    n = len(next(iter(arrays.values())))
+    keep = DUMP_BYTES // (sum(a[0].nbytes for a in arrays.values()) + 8)
+    if keep < n:
+        idx = np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+        arrays = {name: a[idx] for name, a in arrays.items()}
+        arrays["sequence_index"] = idx.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a))
 
 
 def main():
@@ -209,8 +243,6 @@ def main():
     world = int(os.environ.get("WORLD_SIZE", "1"))
 
     if args.impl == "reference":
-        if args.steps > 200:
-            args.steps = 200
         run_reference_arm(args, rank, world)
         return
 
@@ -271,7 +303,8 @@ def main():
     launches = lib.b2t_launch_count() - launches0
     dev_ms = np.array([a.elapsed_time(b) for a, b in ev])
     step_ms = float(dev_ms.sum())
-    stat_host = d_stat[STREAM_WARM + W:].cpu().numpy()
+    stat_host = d_stat[STREAM_WARM + W:STREAM_WARM + W + K].cpu().numpy()     # the K timed steps (d_stat may hold more rows)
+    last_outputs = track_outputs(d_out.cpu().numpy(), stat_host[-1])          # what the last timed step returned
     err = int(stat_host[:, :, L.STAT_ERR].max())
     assert err == 0, "tracker capacity error %d" % err
     algo_bytes = sum(algorithmic_bytes(stat_host[k], esize) for k in range(K)) / K
@@ -374,6 +407,8 @@ def main():
             "wall_s_device_arm": t_wall,
         }
         print(json.dumps(line))
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, last_outputs)
     if world > 1:
         dist.destroy_process_group()
 

@@ -69,7 +69,7 @@ def run_reference(args, rank, world):
     from b200track.w6 import calibrated_state_dict
     sd = calibrated_state_dict(0, args.img, "cuda" if torch.cuda.is_available() else "cpu")
     sd = {k: v.cpu() for k, v in sd.items()}
-    n = max(1, min(args.steps, 30))                              # ~2 s per frame on 32 cores: bounded to about a minute
+    n = args.steps
     w = max(1, min(args.warmup, 2))
     r = BR.run_cpu_arm(sd, args.img, n, w)
     fps = r["value"]
@@ -92,7 +92,7 @@ def run(args):
         return run_reference(args, rank, world)
 
     import torch.distributed as dist
-    from bench import ClockSampler
+    from bench import ClockSampler, track_outputs
     from b200track import _lib as L
     from b200track.detector import DetectorW6
     from b200track.engine import TrackEngine
@@ -166,6 +166,7 @@ def run(args):
     # ---- repeats: the timed region is ~0.4 s; two more runs of the same K steps show the run-to-run spread
     rep_dev = [dev_ms] + [timed_device(K) for _ in range(2)]
     rep_e2e = [e2e_ms] + [timed_e2e(K)[0] for _ in range(2)]
+    last_outputs = track_outputs(*(t.numpy() for t in pipe.flush()))            # what the last timed step returned
     # phase cycles of the last track_step_kernel launch under the pipeline's own load (stat words 16..28, SM clocks; mean over sequences)
     phase_names = ["P0 dets", "P1 lists", "P2 predict", "P3 boxes", "P4 csr1", "P5 lap1", "P6 apply1", "P7 assoc2", "P8 assoc3", "P9 births",
                    "P10 lists", "P11 dedup", "P12 output"]
@@ -302,5 +303,8 @@ def run(args):
             "clocks": clocks,
         }
         print(json.dumps(line))
+        if args.dump_outputs:
+            from bench import dump_outputs
+            dump_outputs(args.dump_outputs, last_outputs)
     if world > 1:
         dist.destroy_process_group()

@@ -3,8 +3,8 @@
 Follows tracker/reid_models/deepsort_reid.py: ``Extractor._preprocess`` :134-146 (crop.astype(float32) / 255 -> cv2.resize to
 64 x 128 -> ToTensor -> Normalize) restated in NumPy, ``Net.forward`` :92-106 with ``reid=True`` (+ ``BasicBlock.forward`` :41-49)
 restated with torch.nn.functional on the checkpoint's tensors (BatchNorm in eval mode, unfolded, fp32).
-tests/test_oracle_reid.py pins both against the UNMODIFIED reference classes -- with seeded weights and, in the build container,
-with the reference's own checkpoint weights/ckpt.t7 (golden features in tests/golden/reid.npz, made by tests/golden/make_golden_reid.py).
+tests/test_oracle_reid.py pins both against what the UNMODIFIED reference classes computed on seeded crops and seeded weights
+(tests/golden/refchecks.npz, made by tests/golden/make_golden_refchecks.py).
 """
 import numpy as np
 import torch

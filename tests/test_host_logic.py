@@ -118,38 +118,17 @@ def test_stream_generator_contract():
 
 
 def test_result_writer_matches_reference_format(tmp_path):
-    """b200track.results against the reference's own save_results (tracker/track.py:247-273), executed from its source when the
-    reference tree is present, else against the documented line formats."""
-    import ast
+    """b200track.results against the files the reference's own save_results (tracker/track.py:247-273) wrote for the same rows
+    (tests/golden/refchecks.npz), and against the documented line formats."""
     import numpy as np
     from b200track.results import format_rows, write_sequence
-    rng = np.random.default_rng(3)
-    frames = []
-    for k in range(4):
-        n = int(rng.integers(1, 6))
-        rows = np.zeros((n, 8))
-        rows[:, 0] = rng.integers(1, 500, n)
-        rows[:, 1:5] = rng.uniform(0, 1280, (n, 4)).round(3)
-        rows[:, 5] = rng.integers(0, 10, n)
-        frames.append(rows)
+    sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
+    from make_golden_refchecks import results_frames
+    g = np.load(os.path.join(ROOT, "tests", "golden", "refchecks.npz"))
+    frames = results_frames()
     for data_type in ("mot17", "default"):
         out = write_sequence(str(tmp_path / ("ours_%s" % data_type) / "seq.txt"), frames, data_type)
-        got = open(out).read()
-        ref_src = os.path.join(os.environ.get("B2T_REFERENCE_ROOT", "/root/reference"), "tracker", "track.py")
-        if os.path.exists(ref_src):
-            tree = ast.parse(open(ref_src).read())
-            fn = next(n for n in tree.body if isinstance(n, ast.FunctionDef) and n.name == "save_results")
-            ns = {"os": os}
-            exec(compile(ast.Module([fn], []), ref_src, "exec"), ns)
-            cwd = os.getcwd()
-            os.chdir(tmp_path)
-            try:
-                results = [(k + 1, [int(r[0]) for r in rows], [r[1:5] for r in rows], [r[5] for r in rows]) for k, rows in enumerate(frames)]
-                ns["save_results"]("ref_%s" % data_type, "seq", results, data_type=data_type)
-                ref = open(os.path.join("tracker", "results", "ref_%s" % data_type, "seq.txt")).read()
-            finally:
-                os.chdir(cwd)
-            assert got == ref
+        assert open(out).read() == str(g["results_" + data_type])
         first = format_rows(1, frames[0][:1], data_type)[0]
         assert first.startswith("1,%d," % int(frames[0][0, 0])) and first.endswith("\n")
         assert first.count(",") == (9 if data_type == "mot17" else 6)

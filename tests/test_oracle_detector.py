@@ -1,15 +1,17 @@
 """not-gpu: the torch oracle of the detector against the committed outputs of the reference's own Model
 (tests/golden/detector_w6.npz) -- pins both oracle/detector.py and the product's graph builder (w6_layers)."""
 import os
+import sys
 
 import numpy as np
-import pytest
 import torch
 
 from b200track.w6 import ANCHORS, STRIDES, conv_shapes, layer_channels, seeded_state_dict, w6_layers
-from oracle import detector as OD, refshim
+from oracle import detector as OD
 
 GOLDEN = os.path.join(os.path.dirname(__file__), "golden", "detector_w6.npz")
+REFCHECKS = os.path.join(os.path.dirname(__file__), "golden", "refchecks.npz")
+sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden"))
 
 
 def test_graph_bookkeeping():
@@ -94,84 +96,64 @@ def test_fold_batchnorm_and_implicit_layers_math():
     assert fold_reference_state_dict(out).keys() == out.keys()        # an already fused dict passes through
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/cfg"), reason="needs the reference tree (build container)")
 def test_fold_training_checkpoint_equals_reference_inference():
-    """The reference's own TRAINING graph (cfg/training/yolov7-w6.yaml: Conv + BN, aux heads, IAuxDetect with implicit layers), with
-    randomised BN statistics, evaluated by the reference in eval mode == the oracle forward on the folded deploy-graph weights."""
+    """The reference's own TRAINING graph (cfg/training/yolov7-w6.yaml: Conv + BN, aux heads, IAuxDetect with implicit layers) on
+    seeded weights for its whole state dict, with seeded BN statistics, evaluated by the reference in eval mode
+    (tests/golden/refchecks.npz) == the oracle forward on the deploy-graph weights folded from that whole state dict."""
     from b200track.w6 import fold_reference_state_dict
-    from oracle import refshim
-    model = refshim.load_detector_model("cfg/training/yolov7-w6.yaml", fuse=False)
-    g = torch.Generator().manual_seed(3)
+    from make_golden_refchecks import stored_shapes, training_state_dict, w6train_image
+    g = np.load(REFCHECKS)
+    anchors = {k.split("/", 1)[1]: g[k] for k in g.files if k.startswith("w6train_anchor/")}
+    sd = training_state_dict(stored_shapes(g["w6train_keys"], g["w6train_key_shapes"]), anchors)
+    assert len(sd) == len(g["w6train_keys"]) and any(k.startswith("model.121.bn.") for k in sd) and any(".m2." in k for k in sd)
+    folded = fold_reference_state_dict(sd)
     with torch.no_grad():
-        for m in model.modules():
-            if isinstance(m, torch.nn.BatchNorm2d):
-                m.running_mean.copy_(torch.randn(m.running_mean.shape, generator=g) * 0.1)
-                m.running_var.copy_(torch.rand(m.running_var.shape, generator=g) * 0.5 + 0.75)
-                m.weight.copy_(torch.rand(m.weight.shape, generator=g) * 0.5 + 1.2)
-                m.bias.copy_(torch.randn(m.bias.shape, generator=g) * 0.1)
-    img = torch.rand((1, 3, 128, 128), generator=g)
-    with torch.no_grad():
-        ref = model(img)[0]
-    folded = fold_reference_state_dict(model.state_dict())
-    with torch.no_grad():
-        got = OD.forward(w6_layers(), folded, img, ANCHORS, STRIDES)
-    assert got.shape == ref.shape
-    assert torch.allclose(got, ref, rtol=2e-3, atol=2e-3), float((got - ref).abs().max())
+        got = OD.forward(w6_layers(), folded, w6train_image(), ANCHORS, STRIDES)
+    assert tuple(got.shape) == tuple(g["w6train_shape"])
+    np.testing.assert_allclose(got[0, g["w6train_rows"]].numpy(), g["w6train_pred_rows"], rtol=2e-3, atol=2e-3)
+    np.testing.assert_allclose(got[0, :, 4].numpy(), g["w6train_obj"], rtol=2e-3, atol=2e-3)
 
 
-def test_pickled_reference_checkpoint_is_converted_and_loaded(tmp_path):
-    """models/experimental.py:83-106 loads a pickled nn.Module.  The drop-in attempt_load refuses such a file with a message that
-    names tools/export_state_dict.py; the converter (run with the reference on sys.path) writes a state dict that the drop-in
-    loader folds to exactly the fused weights the reference's own fuse() produces.  Build container only (needs /root/reference)."""
+def test_pickled_checkpoint_is_refused_and_converted(tmp_path):
+    """The reference's checkpoints pickle the whole nn.Module (its models/experimental.py:83-106).  The drop-in attempt_load refuses
+    such a file with a message that names tools/export_state_dict.py, and the converter, pointed at the package that defines the
+    pickled classes (a stand-in ``models.yolo.Model`` under tmp_path), writes the module's floating-point state dict."""
     import subprocess
-    import sys
-    if not refshim.available():
-        pytest.skip("reference tree not present")
-    ckpt, fused_pt, out = tmp_path / "w6_pickled.pt", tmp_path / "w6_fused.pt", tmp_path / "w6_state.pt"
-    stubs = ("import sys, types\n"
-             "for n in ('matplotlib', 'matplotlib.pyplot', 'seaborn'):\n"
-             "    m = types.ModuleType(n); m.use = lambda *a, **k: None; m.rc = lambda *a, **k: None; sys.modules.setdefault(n, m)\n")
-    make = stubs + ("import os, copy, torch\nos.chdir(%r); sys.path.insert(0, %r)\nfrom models.yolo import Model\n"
-                    "torch.manual_seed(3)\nmodel = Model('cfg/deploy/yolov7-w6.yaml', ch=3, nc=80).float().eval()\n"
-                    "with torch.no_grad():\n"
-                    "    for m in model.modules():\n"
-                    "        if isinstance(m, torch.nn.BatchNorm2d):\n"
-                    "            m.running_mean.normal_(0, 0.1); m.running_var.uniform_(0.5, 1.5); m.weight.normal_(1, 0.1); m.bias.normal_(0, 0.1)\n"
-                    "torch.save({'model': model, 'ema': None, 'epoch': -1}, %r)\n"
-                    "torch.save(copy.deepcopy(model).fuse().state_dict(), %r)\n" % (refshim.REF_ROOT, refshim.REF_ROOT, str(ckpt), str(fused_pt)))
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    (tmp_path / "models").mkdir()
+    (tmp_path / "models" / "__init__.py").write_text("")
+    (tmp_path / "models" / "yolo.py").write_text(
+        "import torch\n\nclass Model(torch.nn.Module):\n    def __init__(self):\n        super().__init__()\n"
+        "        self.conv = torch.nn.Conv2d(3, 8, 3)\n        self.bn = torch.nn.BatchNorm2d(8)\n")
+    ckpt, expect, out = tmp_path / "pickled.pt", tmp_path / "expect.pt", tmp_path / "state.pt"
+    make = ("import sys, torch\nsys.path.insert(0, %r)\nfrom models.yolo import Model\ntorch.manual_seed(3)\nm = Model()\n"
+            "torch.save({'model': m, 'ema': None, 'epoch': -1}, %r)\ntorch.save(m.state_dict(), %r)\n" % (str(tmp_path), str(ckpt), str(expect)))
     r = subprocess.run([sys.executable, "-c", make], capture_output=True, text=True)
     assert r.returncode == 0, r.stderr[-2000:]
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    pkg = os.path.join(root, "yolov7-tracker_b200")
     code = ("import sys; sys.path.insert(0, %r); from models.experimental import attempt_load\n"
-            "try:\n    attempt_load(%r, map_location='cpu')\nexcept RuntimeError as e:\n    print('MSG', str(e))\n" % (pkg, str(ckpt)))
+            "try:\n    attempt_load(%r, map_location='cpu')\nexcept RuntimeError as e:\n    print('MSG', str(e))\n"
+            % (os.path.join(root, "yolov7-tracker_b200"), str(ckpt)))
     r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True)
-    assert "tools/export_state_dict.py" in r.stdout, r.stdout + r.stderr
-    conv = stubs + "sys.argv = ['export_state_dict.py', '--reference', %r, '--weights', %r, '--out', %r]\nimport runpy; runpy.run_path(%r, run_name='__main__')\n" % (
-        refshim.REF_ROOT, str(ckpt), str(out), os.path.join(root, "tools", "export_state_dict.py"))
-    r = subprocess.run([sys.executable, "-c", conv], capture_output=True, text=True)        # (matplotlib / seaborn are absent from this image: stubbed)
+    assert "MSG" in r.stdout and "tools/export_state_dict.py" in r.stdout, r.stdout + r.stderr
+    r = subprocess.run([sys.executable, os.path.join(root, "tools", "export_state_dict.py"), "--reference", str(tmp_path),
+                        "--weights", str(ckpt), "--out", str(out)], capture_output=True, text=True)
     assert r.returncode == 0, r.stderr[-2000:]
-    from b200track.w6 import fold_reference_state_dict
-    folded = fold_reference_state_dict(torch.load(str(out), weights_only=True))
-    ref_sd = torch.load(str(fused_pt), weights_only=True)
-    assert len(folded) == 214
-    for k, v in folded.items():
-        assert torch.allclose(v, ref_sd[k].float(), rtol=1e-5, atol=1e-6), k
+    got, ref = torch.load(str(out), weights_only=True), torch.load(str(expect), weights_only=True)
+    assert set(got) == {k for k, v in ref.items() if v.is_floating_point()} and len(got) == 6
+    assert all(torch.equal(got[k], ref[k]) for k in got)
 
 
-@pytest.mark.skipif(not refshim.available(), reason="reference tree not present")
 def test_tiny_oracle_equals_reference_model():
     """YOLOv7-tiny (cfg/deploy/yolov7-tiny.yaml: LeakyReLU convs, MP / SP pools, three-level Detect): the oracle's restatement of the
-    graph against the reference's own ``Model`` (fused, eval, CPU) on the same seeded weights."""
+    graph against the reference's own ``Model`` (fused, eval, CPU) on the same seeded weights (tests/golden/refchecks.npz)."""
     from b200track import tiny
+    from make_golden_refchecks import stored_shapes, tiny_image
+    g = np.load(REFCHECKS)
     sd = tiny.seeded_state_dict(0)
-    model = refshim.load_detector_model("cfg/deploy/yolov7-tiny.yaml")
-    msd = model.state_dict()
-    assert all(k in msd and msd[k].shape == v.shape for k, v in sd.items()), [k for k in sd if k not in msd][:3]
-    model.load_state_dict(sd, strict=False)
-    img = torch.rand((2, 3, 192, 256), generator=torch.Generator().manual_seed(5))
+    msd = stored_shapes(g["tiny_keys"], g["tiny_key_shapes"])
+    assert all(k in msd and msd[k] == tuple(v.shape) for k, v in sd.items()), [k for k in sd if k not in msd][:3]
     with torch.no_grad():
-        ref = model(img)[0]
-        got = OD.forward(tiny.tiny_layers(), sd, img, tiny.ANCHORS, tiny.STRIDES, act="leaky", name_offset=-1)
-    assert ref.shape == got.shape == (2, 3 * (24 * 32 + 12 * 16 + 6 * 8), 85)
-    assert float((ref - got).abs().max()) < 2e-3 and float((ref[..., 4] - got[..., 4]).abs().max()) < 1e-5
+        got = OD.forward(tiny.tiny_layers(), sd, tiny_image(), tiny.ANCHORS, tiny.STRIDES, act="leaky", name_offset=-1).numpy()
+    assert tuple(g["tiny_shape"]) == got.shape == (2, 3 * (24 * 32 + 12 * 16 + 6 * 8), 85)
+    assert float(np.abs(got[:, g["tiny_rows"]] - g["tiny_pred_rows"]).max()) < 2e-3
+    assert float(np.abs(got[..., 4] - g["tiny_obj"]).max()) < 1e-5

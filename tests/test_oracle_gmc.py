@@ -1,5 +1,5 @@
 """Pins oracle/gmc.py (the restatement of tracker/botsort.py:111-235, GMC method 'orb') stage by stage against the cv2 calls the
-reference makes, and end to end against the UNMODIFIED reference class (build container only).  CPU tier."""
+reference makes, and end to end against what the UNMODIFIED reference class computed (tests/golden).  CPU tier."""
 import os
 import sys
 
@@ -13,7 +13,6 @@ for p in (ROOT, os.path.join(ROOT, "yolov7-tracker_b200")):
 
 cv2 = pytest.importorskip("cv2")
 from oracle import gmc as G                      # noqa: E402
-from oracle import refshim                       # noqa: E402
 from b200track.synth import textured_frame      # noqa: E402
 
 
@@ -70,27 +69,23 @@ def test_knn2_equals_bfmatcher():
     assert all(m[0].trainIdx == i1[q] and m[0].distance == b1[q] and m[1].trainIdx == i2[q] and m[1].distance == b2[q] for q, m in enumerate(knn))
 
 
-@pytest.mark.skipif(not refshim.available(), reason="reference tree not present")
 def test_estimate_equals_reference_class():
     """The whole recipe against the reference's own GMC(method='orb', downscale=2).apply over a short moving sequence with
-    detections masked out: same key points, same matches -> the same cv2.estimateAffinePartial2D input -> the same matrix."""
-    ref = refshim.load().botsort.GMC(method='orb', downscale=2)
+    detections masked out (tests/golden/refchecks.npz): same key points, same matches -> the same cv2.estimateAffinePartial2D
+    input -> the same matrix."""
+    sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
+    from make_golden_refchecks import gmc_sequence
+    g = np.load(os.path.join(ROOT, "tests", "golden", "refchecks.npz"))
     orc = G.GMCOracle(estimator="cv2")
     own = G.GMCOracle(estimator="restated")
-    f = textured_frame(11, 720, 1280)
-    dets = np.array([[200, 100, 420, 500, 0.9, 0], [700, 300, 900, 640, 0.7, 1]], np.float32)
-    rng = np.random.default_rng(0)
-    for k in range(4):
-        Hr = ref.apply(f, dets)
+    for k, (f, dets) in enumerate(gmc_sequence()):
+        Hr = g["gmc_H"][k]
         Ho = orc.apply(f, dets)
         Hw = own.apply(f, dets)
         np.testing.assert_allclose(Ho, Hr, rtol=0, atol=1e-9)
         if k:
             # the restated RANSAC (own sampling sequence) against OpenCV's: within the spread of its own random sampling
             assert np.abs(Hw[:, :2] - Hr[:, :2]).max() < 1e-3 and np.abs(Hw[:, 2] - Hr[:, 2]).max() < 0.25, (Hw, Hr)
-        true = (float(rng.uniform(-6, 6)), float(rng.uniform(-6, 6)))
-        f, _ = moved(f, float(rng.uniform(-0.5, 0.5)), 1.0 + float(rng.uniform(-0.004, 0.004)), *true)
-        dets = dets + np.array([true[0], true[1], true[0], true[1], 0, 0], np.float32)
 
 
 def test_oracle_reproduces_committed_reference_golden():

@@ -1,11 +1,9 @@
-"""Pins oracle/reid.py (restatement of tracker/reid_models/deepsort_reid.py) against the UNMODIFIED reference: the committed golden
-features made with the reference's own checkpoint (tests/golden/reid.npz), and -- build container only -- the reference classes run
-live with seeded weights and with weights/ckpt.t7.  CPU tier."""
+"""Pins oracle/reid.py (restatement of tracker/reid_models/deepsort_reid.py) against what the UNMODIFIED reference computed on the
+same seeded crops and weights (tests/golden/refchecks.npz).  CPU tier."""
 import os
 import sys
 
 import numpy as np
-import pytest
 import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -14,58 +12,33 @@ for p in (ROOT, os.path.join(ROOT, "yolov7-tracker_b200")):
         sys.path.insert(0, p)
 from oracle import reid as R  # noqa: E402
 
-REF = os.environ.get("B2T_REFERENCE_ROOT", "/root/reference")
-HAVE_REF = os.path.exists(os.path.join(REF, "weights", "ckpt.t7"))
+GOLDEN = os.path.join(ROOT, "tests", "golden", "refchecks.npz")
 
 
-def _ref_module():
-    sys.path.insert(0, os.path.join(REF, "tracker"))
-    try:
-        from reid_models import deepsort_reid as M
-    finally:
-        sys.path.remove(os.path.join(REF, "tracker"))
-        for k in [k for k in sys.modules if k.startswith("reid_models")]:
-            del sys.modules[k]
-    return M
-
-
-@pytest.mark.skipif(not HAVE_REF, reason="reference tree / checkpoint not present")
 def test_restatement_equals_reference_net_and_preprocess():
-    M = _ref_module()
-    crops = R.seeded_crops(9, 5)
-    ext = M.Extractor(os.path.join(REF, "weights", "ckpt.t7"), use_cuda=False)
-    x_ref = ext._preprocess(crops)
+    """Against tests/golden/refchecks.npz (tests/golden/make_golden_refchecks.py): the reference Extractor's _preprocess of the same
+    seeded crops, and the reference's own Net on the seeded weights in eval mode, in training mode (the extractor's mode), and in
+    eval mode after that training-mode call updated the BatchNorm buffers."""
+    sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
+    from make_golden_refchecks import REID_CROPS
+    g = np.load(GOLDEN)
+    crops = R.seeded_crops(*REID_CROPS)
     x = R.preprocess(crops)
-    assert x.shape == x_ref.shape and float((x - x_ref).abs().max()) < 2e-6                  # cv2.resize on float data, restated
-    sd = {k: v.float() for k, v in ext.net.state_dict().items() if v.dtype.is_floating_point}
-    assert ext.net.training                                     # the quirk: the reference never switches its extractor to eval()
-    with torch.no_grad():
-        f = R.forward(sd, x, batch_stats=True)                   # (before the reference call: that one also updates the running buffers)
-        f_ref = ext.net(x_ref)
-        f_eval_ref = ext.net.eval()(x_ref)
-        ext.net.train()
-    assert float((f - f_ref).abs().max()) < 2e-5
-    sd_after = {k: v.float() for k, v in ext.net.state_dict().items() if v.dtype.is_floating_point}
-    with torch.no_grad():
-        assert float((R.forward(sd_after, x, batch_stats=False) - f_eval_ref).abs().max()) < 2e-5
-    # seeded weights (what the GPU tier uses) through the reference's own Net
-    net = M.Net(reid=True).eval()
+    assert tuple(x.shape) == tuple(g["reid_x_shape"])
+    xs = x.numpy()                                              # cv2.resize on float data, restated
+    assert float(np.abs(xs.reshape(-1)[g["reid_x_index"]] - g["reid_x_values"]).max()) < 2e-6
+    assert np.all(np.abs(xs.astype(np.float64).sum(axis=(1, 2, 3)) - g["reid_x_sums"]) < 2e-6 * xs[0].size)
+    assert bool(g["reid_extractor_training"])                   # the quirk: the reference never switches its extractor to eval()
     seeded = R.seeded_state_dict(3)
-    missing = net.load_state_dict(seeded, strict=False)
-    assert not [k for k in missing.missing_keys if "classifier" not in k and "num_batches_tracked" not in k] and not missing.unexpected_keys
+    ref_keys = set(g["reid_net_keys"].tolist())
+    assert not [k for k in ref_keys - set(seeded) if "classifier" not in k and "num_batches_tracked" not in k] and not set(seeded) - ref_keys
     with torch.no_grad():
-        assert float((net(x) - R.forward(seeded, x, batch_stats=False)).abs().max()) < 2e-5
-        assert float((net.train()(x) - R.forward(seeded, x, batch_stats=True)).abs().max()) < 2e-5
-
-
-@pytest.mark.skipif(not HAVE_REF, reason="reference tree / checkpoint not present")
-def test_golden_features_reproduce_with_the_checkpoint():
-    g = np.load(os.path.join(ROOT, "tests", "golden", "reid.npz"))
-    ck = torch.load(os.path.join(REF, "weights", "ckpt.t7"), map_location="cpu", weights_only=False)["net_dict"]
-    sd = {k: v.float() for k, v in ck.items() if v.dtype.is_floating_point}
+        assert float(np.abs(R.forward(seeded, x, batch_stats=False).numpy() - g["reid_eval"]).max()) < 2e-5
+        assert float(np.abs(R.forward(seeded, x, batch_stats=True).numpy() - g["reid_train"]).max()) < 2e-5
+    sd_after = dict(seeded)
+    sd_after.update({k.split("/", 1)[1]: torch.from_numpy(g[k]) for k in g.files if k.startswith("reid_after/")})
     with torch.no_grad():
-        f = R.forward(sd, R.preprocess(R.seeded_crops(int(g["seed"]), int(g["n"]))), batch_stats=True)
-    np.testing.assert_allclose(f.numpy(), g["features"], rtol=0, atol=2e-5)
+        assert float(np.abs(R.forward(sd_after, x, batch_stats=False).numpy() - g["reid_eval_after"]).max()) < 2e-5
 
 
 def test_seeded_network_is_well_conditioned():

@@ -28,7 +28,7 @@ extern "C" {
 
 enum { B2T_F32 = 0, B2T_F64 = 1 };
 enum { B2T_FMT_XYAH = 0, B2T_FMT_XYWH = 1, B2T_FMT_NSA = 2 };
-enum { B2T_SORT = 0, B2T_BYTETRACK = 1, B2T_BOTSORT = 2 };
+enum { B2T_SORT = 0, B2T_BYTETRACK = 1, B2T_BOTSORT = 2, B2T_CBIOU = 3 };
 enum { B2T_OK = 0, B2T_EINVAL = -1, B2T_ECUDA = -2, B2T_ECAPACITY = -3, B2T_ENOTBUILT = -4 };
 /* 16-bit activation / weight type of the detector branch.  Both feed tcgen05 kind::f16 at the same rate with fp32
  * accumulation; fp16 (the reference's own GPU half mode, detect.py:41) carries 3 more mantissa bits than bf16. */
@@ -79,11 +79,16 @@ int b2t_lap_solve(int dtype, const void* cost, int n, int m, int ld, double thre
 /* ---------------------------------------------------------------- fused trackers
  * One object = S independent video sequences advanced together, one CTA per sequence per frame:
  *   BaseTracker.update tracker/basetrack.py:368-487, ByteTrack.update tracker/bytetrack.py:41-204,
- *   BoTSORT.update tracker/botsort.py:313-493. */
+ *   BoTSORT.update tracker/botsort.py:313-493, C_BIoUTracker.update tracker/c_biou_tracker.py:218-353.
+ * B2T_CBIOU (cascaded buffered IoU, no Kalman filter) reads conf_thresh, track_buffer and frame_rate and ignores fmt, iou_thresh and
+ * use_gmc.  It needs dtype = B2T_F64 (B2T_EINVAL otherwise: the reference's IoU is float64 and there is no Kalman state to shrink) and
+ * rejects predict_only (the reference's update_without_detection needs a Kalman filter).  Its lost tracks are never pruned (as in the
+ * reference), so cap bounds the tracks a sequence can ever hold at once, lost ones included: an overflow is the sticky capacity
+ * error, never a dropped track.  The per-slot record it keeps is documented with b2t_tracker_read_slot. */
 typedef struct b2t_tracker b2t_tracker;
 
 typedef struct b2t_tracker_config {
-    int kind;          /* B2T_SORT / B2T_BYTETRACK / B2T_BOTSORT */
+    int kind;          /* B2T_SORT / B2T_BYTETRACK / B2T_BOTSORT / B2T_CBIOU */
     int dtype;         /* B2T_F32 / B2T_F64 */
     int fmt;           /* Kalman format */
     int n_seq;         /* sequences per launch */
@@ -118,12 +123,16 @@ int b2t_tracker_step_host(b2t_tracker* t, const float* dets_host, const int* det
                           const double* warps_host, const int* id_base_host, double* out_host, int out_rows,
                           int* stat_host, int predict_only, void* stream);
 /* One sequence's ordered list of tracked (which = 0) or lost (which = 1) tracks -- BaseTracker.tracked_stracks / .lost_stracks,
- * basetrack.py:358-360 -- as rows of b2t_tracker_list_cols() = 13 doubles on the HOST: id, tlwh[4] (STrack.tlwh of the Kalman mean),
+ * basetrack.py:358-360 -- as rows of b2t_tracker_list_cols() = 13 doubles on the HOST: id, tlwh[4] (STrack.tlwh of the Kalman mean;
+ * B2T_CBIOU: the last matched detection box, C_BIoUSTrack.tlwh),
  * cls, score, slot, state, is_activated, tracklet_len, start_frame, frame_id.  *n_host = list length (rows beyond max_rows are not copied).
  * Synchronises the stream. */
 int b2t_tracker_list_cols(void);
 int b2t_tracker_read_list(b2t_tracker* t, int seq, int which, double* rows_host, int max_rows, int* n_host, void* stream);
-/* Copies one slot's Kalman state to the host as float64: mean[8], cov[64] (lazy STrack.mean/.cov). */
+/* Copies one slot's Kalman state to the host as float64: mean[8], cov[64] (lazy STrack.mean/.cov).
+ * B2T_CBIOU keeps another record in the same 72 doubles r = mean[0..8) ++ cov[0..64): r[0] history length n (1..6), r[1]
+ * time_since_update, r[8..32) the last n matched tlwh boxes oldest first, r[32..36) motion_state1, r[36..40) motion_state2 (tlwh);
+ * the rest is unused.  Box values are float32 numbers. */
 int b2t_tracker_read_slot(b2t_tracker* t, int seq, int slot, double* mean_host, double* cov_host, void* stream);
 
 /* ---------------------------------------------------------------- detector: conv + bias + SiLU (tcgen05 / TMA)

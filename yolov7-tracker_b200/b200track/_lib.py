@@ -13,7 +13,7 @@ LIB_PATH = os.environ.get("B2T_LIB_PATH") or os.path.join(HERE, "libb200track.so
 
 F32, F64 = 0, 1
 FMT_XYAH, FMT_XYWH, FMT_NSA = 0, 1, 2
-SORT, BYTETRACK, BOTSORT = 0, 1, 2
+SORT, BYTETRACK, BOTSORT, CBIOU = 0, 1, 2, 3
 FLAG_MEAN_F32, FLAG_NOT_TRACKED = 1, 2
 ACT_BF16, ACT_F16 = 0, 1
 OUT_COLS, STAT_WORDS, STAT_PHASE0, STAT_SUB0 = 8, 64, 16, 32
@@ -21,7 +21,7 @@ GMC_STAT_WORDS, GMC_FIRST_FRAME, GMC_FEW_POINTS, GMC_TRUNCATED = 8, 1, 2, 4
 (STAT_NOUT, STAT_NEXT_ID, STAT_NTRACKED, STAT_NLOST, STAT_ERR, STAT_FRAME, STAT_NPOOL, STAT_NBIRTH,
  STAT_NHI, STAT_NLO, STAT_NEDGE, STAT_NMATCH0) = range(12)
 FMT_BY_NAME = {"default": FMT_XYAH, "botsort": FMT_XYWH, "strongsort": FMT_NSA}
-KIND_BY_NAME = {"sort": SORT, "bytetrack": BYTETRACK, "botsort": BOTSORT}
+KIND_BY_NAME = {"sort": SORT, "bytetrack": BYTETRACK, "botsort": BOTSORT, "c_biou": CBIOU}
 
 
 class B2TError(RuntimeError):

@@ -25,6 +25,9 @@ class TrackEngine:
         self.device = torch.device(device)
         if self.device.type == "cuda" and self.device.index is None:
             self.device = torch.device("cuda", torch.cuda.current_device())
+        if kind == "c_biou":
+            # C-BIoU has no Kalman filter (the format is never read) and runs in float64 only, like the reference's buffered IoU
+            kalman_format, dtype = "default", "f64"
         if kalman_format is None:
             kalman_format = "botsort" if kind == "botsort" else "default"      # track.py:68-69
         self.kind, self.kalman_format = kind, kalman_format
@@ -195,12 +198,23 @@ class TrackEngine:
         return rows[:n.value].copy()
 
     def read_slot(self, seq, slot):
+        """The slot's 72-double record as (mean[8], cov[8, 8]): the Kalman state, or for kind c_biou the record documented in
+        csrc/b2t_cbiou.cuh (see cbiou_record)."""
         mean = np.zeros(8); cov = np.zeros((8, 8))
         with torch.cuda.device(self.device):
             rc = self.lib.b2t_tracker_read_slot(self.handle, int(seq), int(slot), mean.ctypes.data_as(C.c_void_p),
                                                 cov.ctypes.data_as(C.c_void_p), self._stream())
         L.check(self.lib, rc)
         return mean, cov
+
+    def cbiou_record(self, seq, slot):
+        """Kind c_biou: the slot's record as a dict -- history (n, 4) tlwh oldest first, motion_state1 / motion_state2 (4,) tlwh,
+        time_since_update -- float32 boxes as the reference keeps them."""
+        mean, cov = self.read_slot(seq, slot)
+        r = np.concatenate([mean, cov.reshape(-1)])
+        n = int(r[0])
+        return dict(history=r[8:8 + 4 * n].reshape(n, 4).astype(np.float32), motion_state1=r[32:36].astype(np.float32),
+                    motion_state2=r[36:40].astype(np.float32), time_since_update=int(r[1]))
 
 
 # ------------------------------------------------------------------ op-level helpers (device tensors)

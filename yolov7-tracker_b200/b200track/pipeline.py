@@ -12,6 +12,8 @@ post-processed while frame t's forward runs: the detect stream never idles betwe
 staging, the stem input, the head maps and the NMS output of each detector) are guarded by events.  ``step()`` returns the tracks of
 the PREVIOUS call (one frame of latency, same results); ``flush()`` returns the last ones.
 """
+import gc
+
 import torch
 
 from . import _lib as L
@@ -57,6 +59,10 @@ class TrackingPipeline:
         self._capture()
 
     def _capture(self):
+        # Collect dead objects first: an unreachable detector (its op closures hold it in a reference cycle) is otherwise freed by
+        # whichever garbage collection happens to run next -- possibly inside a capture below, where its plans' cudaFree would
+        # invalidate the graph.  torch.cuda.graph no longer collects on entry.
+        gc.collect()
         torch.cuda.synchronize()
         for i, det in enumerate(self.dets):
             with torch.cuda.stream(self.s_det):

@@ -54,6 +54,31 @@ def make_stream(seed, n_frames, n_obj=300, img=1280, miss=0.05, warp_sigma=0.0):
     return frames, warps
 
 
+def make_vanish_stream(seed, n_frames, per_frame=3, img=1280):
+    """Seeded stream of short-lived objects: every frame starts `per_frame` new objects that move for 3..8 frames and vanish
+    (C-BIoU never prunes its lost tracks, so this stream grows the lost list without bound).
+    Per frame an (n, 6) float32 [x1, y1, x2, y2, score, cls] array, integer-rounded boxes, sorted by descending score."""
+    rng = np.random.default_rng(seed)
+    objs = []
+    frames = []
+    for f in range(n_frames):
+        for _ in range(per_frame):
+            cx, cy = rng.uniform(100, img - 100, 2)
+            w, h = rng.uniform(20, 80), rng.uniform(40, 160)
+            objs.append([cx, cy, w, h, rng.normal(0, 3), rng.normal(0, 3), f + int(rng.integers(3, 9)), float(rng.integers(0, 3))])
+        rows = []
+        for o in objs:
+            if o[6] <= f:
+                continue
+            o[0] += o[4]; o[1] += o[5]
+            box = np.round(np.clip([o[0] - o[2] / 2, o[1] - o[3] / 2, o[0] + o[2] / 2, o[1] + o[3] / 2] + rng.normal(0, 1, 4), 0, img))
+            rows.append([*box, rng.uniform(0.3, 0.95), o[7]])
+        objs = [o for o in objs if o[6] > f]
+        d = np.array(rows, np.float32).reshape(-1, 6)
+        frames.append(np.ascontiguousarray(d[np.argsort(-d[:, 4], kind="stable")]))
+    return frames
+
+
 def stream_digest(frames):
     """sha1 of the raw bytes: stored with golden fixtures to detect generator drift."""
     hsh = hashlib.sha1()

@@ -394,6 +394,92 @@ B2T_DEVNI void apply_matches(StepCtx<T>& c, const int* rows, int n, const float*
 
 #define B2T_PHASE(idx) do { if (tid == 0) { const long long now_ = phase_clock(); stat[STAT_PHASE0 + (idx)] = (int)(now_ - tprev); tprev = now_; } } while (0)
 
+struct FrameLists { int nt, nl, nout, nfree; };
+
+// P9-P11 of a frame, shared by every kind: list algebra (bytetrack.py:186-193), remove_duplicate_stracks (basetrack.py:563-576),
+// the output rows of the activated tracks and the free list.  box(slot, tlbr, out[4]) writes a track's box as tlbr (duplicate
+// test) or tlwh (output rows): the Kalman kinds read it from the mean, C-BIoU from its last matched detection.
+// On entry the states of this frame are final, sm.births[0..nbirth) / sm.refind[0..nref) / sm.lost_now[0..nlostnow) hold slots.
+template <class T, class BoxFn>
+B2T_DEV FrameLists finish_lists(StepCtx<T>& c, BoxFn box, int n_tracked0, int n_lost0, int nbirth, int nref, int nlostnow,
+                                double* out, int out_rows, int* err, int* stat, long long& tprev) {
+    StepSmem<T>& sm = c.sm;
+    SeqView<T>& v = c.v;
+    const StepParams& p = c.p;
+    const int tid = (int)threadIdx.x, nthr = (int)blockDim.x;
+    const int cap = v.cap;
+    const int f = c.f;
+    // ---- P9: list algebra (bytetrack.py:186-193)
+    int nt1 = block_compact(n_tracked0, [&](int k) { return v.state[v.tracked[k]] == ST_TRACKED; }, sm.ut, sm.misc);
+    for (int k = tid; k < nt1; k += nthr) sm.ntr[k] = v.tracked[sm.ut[k]];
+    for (int k = tid; k < nbirth; k += nthr) sm.ntr[nt1 + k] = sm.births[k];
+    for (int k = tid; k < nref; k += nthr) sm.ntr[nt1 + nbirth + k] = sm.refind[k];
+    nt1 += nbirth + nref;
+    if (nt1 > cap) { nt1 = cap; if (tid == 0) *err |= ERR_SLOTS; }
+    // old lost entries that were not re-found and whose id was not in the removed list before this frame
+    int nl1 = block_compact(n_lost0, [&](int k) { const int s = v.lost[k];
+        return v.state[s] != ST_TRACKED && !(v.removed_at[s] != 0 && v.removed_at[s] < f); }, sm.ut, sm.misc);
+    for (int k = tid; k < nl1; k += nthr) sm.nlo[k] = v.lost[sm.ut[k]];
+    __syncthreads();
+    const int nl_add = block_compact(nlostnow, [&](int k) { const int s = sm.lost_now[k];
+        return !(v.removed_at[s] != 0 && v.removed_at[s] < f); }, sm.ut, sm.misc);
+    for (int k = tid; k < nl_add; k += nthr) sm.nlo[nl1 + k] = sm.lost_now[sm.ut[k]];
+    nl1 += nl_add;
+    __syncthreads();
+
+    B2T_PHASE(10);
+    // ---- P10: remove_duplicate_stracks (basetrack.py:563-576)
+    for (int k = tid; k < cap; k += nthr) { sm.dupa[k] = 0; sm.dupb[k] = 0; }
+    for (int k = tid; k < nt1; k += nthr) box(sm.ntr[k], true, sm.rowbox + 4 * k);
+    for (int k = tid; k < nl1; k += nthr) box(sm.nlo[k], true, sm.colbox + 4 * k);
+    __syncthreads();
+    if (nt1 > 0 && nl1 > 0) {
+        const bool ok = build_csr<T>(v, sm, nt1, nl1, (T)p.t_dup);
+        if (!ok && tid == 0) *err |= ERR_EDGES;
+        const LapCsr<T> g = step_csr<T>(c);
+        for (int i = warp_id(); i < nt1; i += num_warps()) {
+            const int sa = sm.ntr[i];
+            const int timep = v.frame_id[sa] - v.start_frame[sa];
+            const int es = sm.rstart[i], ec = sm.rcnt[i];
+            const int* ecol = g.cols(es, ec);
+            for (int e = lane_id(); e < ec; e += 32) {
+                const int q = ecol[e];
+                if (q < 0) continue;
+                const int sb = sm.nlo[q];
+                const int timeq = v.frame_id[sb] - v.start_frame[sb];
+                if (timep > timeq) sm.dupb[q] = 1; else sm.dupa[i] = 1;
+            }
+        }
+        __syncthreads();
+    }
+    const int nt2 = block_compact(nt1, [&](int k) { return sm.dupa[k] == 0; }, sm.ut, sm.misc);
+    for (int k = tid; k < nt2; k += nthr) v.tracked[k] = sm.ntr[sm.ut[k]];
+    const int nl2 = block_compact(nl1, [&](int k) { return sm.dupb[k] == 0; }, sm.ut, sm.misc);
+    for (int k = tid; k < nl2; k += nthr) v.lost[k] = sm.nlo[sm.ut[k]];
+    for (int k = tid; k < cap; k += nthr) sm.used[k] = 0;
+    __syncthreads();
+
+    B2T_PHASE(11);
+    // ---- P11: output rows (activated tracks, bytetrack.py:204) and the free list
+    for (int k = tid; k < nt2; k += nthr) sm.used[v.tracked[k]] = 1;
+    for (int k = tid; k < nl2; k += nthr) sm.used[v.lost[k]] = 1;
+    __syncthreads();
+    int nout = block_compact(nt2, [&](int k) { return v.activated[v.tracked[k]] != 0; }, sm.ut, sm.misc);
+    if (nout > out_rows) { nout = out_rows; if (tid == 0) *err |= ERR_OUT; }
+    for (int k = tid; k < nout; k += nthr) {
+        const int s = v.tracked[sm.ut[k]];
+        T b[4];
+        box(s, false, b);
+        double* o = out + (size_t)k * OUT_COLS;
+        o[0] = (double)v.tid[s];
+        o[1] = (double)b[0]; o[2] = (double)b[1]; o[3] = (double)b[2]; o[4] = (double)b[3];
+        o[5] = (double)v.cls[s]; o[6] = (double)v.score[s]; o[7] = (double)s;
+    }
+    const int nfree2 = block_compact(cap, [&](int k) { return sm.used[k] == 0; }, v.freelist, sm.misc);
+    B2T_PHASE(12);
+    return FrameLists{nt2, nl2, nout, nfree2};
+}
+
 template <class T>
 B2T_DEV void track_step_cta(const TrackState& st, const StepParams& prm, int seq, const float* dets_all,
                             const int* det_count, const double* warps, const int* id_base, double* out_all,
@@ -640,77 +726,14 @@ B2T_DEV void track_step_cta(const TrackState& st, const StepParams& prm, int seq
     }
 
     B2T_PHASE(9);
-    // ---- P9: list algebra (bytetrack.py:186-193)
-    int nt1 = block_compact(n_tracked0, [&](int k) { return v.state[v.tracked[k]] == ST_TRACKED; }, sm.ut, sm.misc);
-    for (int k = tid; k < nt1; k += nthr) sm.ntr[k] = v.tracked[sm.ut[k]];
-    for (int k = tid; k < nbirth; k += nthr) sm.ntr[nt1 + k] = sm.births[k];
-    for (int k = tid; k < nref; k += nthr) sm.ntr[nt1 + nbirth + k] = sm.refind[k];
-    nt1 += nbirth + nref;
-    if (nt1 > cap) { nt1 = cap; if (tid == 0) *err |= ERR_SLOTS; }
-    // old lost entries that were not re-found and whose id was not in the removed list before this frame
-    int nl1 = block_compact(n_lost0, [&](int k) { const int s = v.lost[k];
-        return v.state[s] != ST_TRACKED && !(v.removed_at[s] != 0 && v.removed_at[s] < f); }, sm.ut, sm.misc);
-    for (int k = tid; k < nl1; k += nthr) sm.nlo[k] = v.lost[sm.ut[k]];
-    __syncthreads();
-    const int nl_add = block_compact(nlostnow, [&](int k) { const int s = sm.lost_now[k];
-        return !(v.removed_at[s] != 0 && v.removed_at[s] < f); }, sm.ut, sm.misc);
-    for (int k = tid; k < nl_add; k += nthr) sm.nlo[nl1 + k] = sm.lost_now[sm.ut[k]];
-    nl1 += nl_add;
-    __syncthreads();
-
-    B2T_PHASE(10);
-    // ---- P10: remove_duplicate_stracks (basetrack.py:563-576)
-    for (int k = tid; k < cap; k += nthr) { sm.dupa[k] = 0; sm.dupb[k] = 0; }
-    fill_track_boxes<T>(v, p.fmt, sm.ntr, nt1, sm.rowbox);
-    fill_track_boxes<T>(v, p.fmt, sm.nlo, nl1, sm.colbox);
-    __syncthreads();
-    if (nt1 > 0 && nl1 > 0) {
-        const bool ok = build_csr<T>(v, sm, nt1, nl1, (T)p.t_dup);
-        if (!ok && tid == 0) *err |= ERR_EDGES;
-        const LapCsr<T> g = step_csr<T>(c);
-        for (int i = warp_id(); i < nt1; i += num_warps()) {
-            const int sa = sm.ntr[i];
-            const int timep = v.frame_id[sa] - v.start_frame[sa];
-            const int es = sm.rstart[i], ec = sm.rcnt[i];
-            const int* ecol = g.cols(es, ec);
-            for (int e = lane_id(); e < ec; e += 32) {
-                const int q = ecol[e];
-                if (q < 0) continue;
-                const int sb = sm.nlo[q];
-                const int timeq = v.frame_id[sb] - v.start_frame[sb];
-                if (timep > timeq) sm.dupb[q] = 1; else sm.dupa[i] = 1;
-            }
-        }
-        __syncthreads();
-    }
-    const int nt2 = block_compact(nt1, [&](int k) { return sm.dupa[k] == 0; }, sm.ut, sm.misc);
-    for (int k = tid; k < nt2; k += nthr) v.tracked[k] = sm.ntr[sm.ut[k]];
-    const int nl2 = block_compact(nl1, [&](int k) { return sm.dupb[k] == 0; }, sm.ut, sm.misc);
-    for (int k = tid; k < nl2; k += nthr) v.lost[k] = sm.nlo[sm.ut[k]];
-    for (int k = tid; k < cap; k += nthr) sm.used[k] = 0;
-    __syncthreads();
-
-    B2T_PHASE(11);
-    // ---- P11: output rows (activated tracks, bytetrack.py:204) and the free list
-    for (int k = tid; k < nt2; k += nthr) sm.used[v.tracked[k]] = 1;
-    for (int k = tid; k < nl2; k += nthr) sm.used[v.lost[k]] = 1;
-    __syncthreads();
-    int nout = block_compact(nt2, [&](int k) { return v.activated[v.tracked[k]] != 0; }, sm.ut, sm.misc);
-    if (nout > out_rows) { nout = out_rows; if (tid == 0) *err |= ERR_OUT; }
-    for (int k = tid; k < nout; k += nthr) {
-        const int s = v.tracked[sm.ut[k]];
-        T box[4];
-        mean_to_tlwh<T>(p.fmt, v.mean + (size_t)s * 8, (v.flags[s] & 1) != 0, box);
-        double* o = out + (size_t)k * OUT_COLS;
-        o[0] = (double)v.tid[s];
-        o[1] = (double)box[0]; o[2] = (double)box[1]; o[3] = (double)box[2]; o[4] = (double)box[3];
-        o[5] = (double)v.cls[s]; o[6] = (double)v.score[s]; o[7] = (double)s;
-    }
-    const int nfree2 = block_compact(cap, [&](int k) { return sm.used[k] == 0; }, v.freelist, sm.misc);
-    B2T_PHASE(12);
+    auto kalman_box = [&](int s, bool tlbr, T* box) {
+        if (tlbr) mean_to_tlbr<T>(p.fmt, v.mean + (size_t)s * 8, (v.flags[s] & 1) != 0, box);
+        else mean_to_tlwh<T>(p.fmt, v.mean + (size_t)s * 8, (v.flags[s] & 1) != 0, box);
+    };
+    const FrameLists fl = finish_lists<T>(c, kalman_box, n_tracked0, n_lost0, nbirth, nref, nlostnow, out, out_rows, err, stat, tprev);
     if (tid == 0) {
-        v.ctrl[CTRL_NTRACKED] = nt2; v.ctrl[CTRL_NLOST] = nl2; v.ctrl[CTRL_NFREE] = nfree2; v.ctrl[CTRL_ERR] = *err;
-        stat[STAT_NOUT] = nout; stat[STAT_NEXT_ID] = v.ctrl[CTRL_NEXT_ID]; stat[STAT_NTRACKED] = nt2; stat[STAT_NLOST] = nl2;
+        v.ctrl[CTRL_NTRACKED] = fl.nt; v.ctrl[CTRL_NLOST] = fl.nl; v.ctrl[CTRL_NFREE] = fl.nfree; v.ctrl[CTRL_ERR] = *err;
+        stat[STAT_NOUT] = fl.nout; stat[STAT_NEXT_ID] = v.ctrl[CTRL_NEXT_ID]; stat[STAT_NTRACKED] = fl.nt; stat[STAT_NLOST] = fl.nl;
         stat[STAT_ERR] = *err; stat[STAT_FRAME] = f; stat[STAT_NPOOL] = npool; stat[STAT_NBIRTH] = nbirth;
         stat[STAT_NHI] = nhi; stat[STAT_NLO] = nlo; stat[STAT_NEDGE] = sm.misc[50]; stat[STAT_NMATCH0] = nmatch0;
     }

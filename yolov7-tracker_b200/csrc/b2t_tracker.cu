@@ -1,11 +1,12 @@
 // b2t_tracker.cu -- kernels + C ABI (include/b200track.h) for the association branch:
 // batched Kalman ops, "+1" IoU cost, thresholded exact assignment and the fused per-frame
-// SORT / ByteTrack / BoT-SORT step.  Compiled for sm_100a with --fmad=false (see b2t_iou.cuh).
+// SORT / ByteTrack / BoT-SORT step and the fused C-BIoU step.  Compiled for sm_100a with --fmad=false (see b2t_iou.cuh).
 #include <string>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
 #include "b2t_step.cuh"
+#include "b2t_cbiou.cuh"
 #include "../../include/b200track.h"
 
 using namespace b2t;
@@ -229,6 +230,15 @@ track_step_kernel(TrackState st, StepParams prm, const float* dets, const int* d
     track_step_cta<T>(st, prm, (int)blockIdx.x, dets, det_count, warps, id_base, out, out_rows, stat, smem_raw);
 }
 
+// C-BIoU (b2t_cbiou.cuh): its own kernel, so that the three Kalman kinds above compile exactly as before
+template <class T>
+__global__ void __launch_bounds__(512, 1)
+cbiou_step_kernel(TrackState st, StepParams prm, const float* dets, const int* det_count, const int* id_base, double* out,
+                  int out_rows, int* stat) {
+    B2T_DYN_SMEM(smem_raw);
+    cbiou_step_cta<T>(st, prm, (int)blockIdx.x, dets, det_count, id_base, out, out_rows, stat, smem_raw);
+}
+
 __global__ void track_reset_kernel(TrackState st) {
     const int s = (int)blockIdx.x;
     const size_t o = (size_t)s * st.cap;
@@ -250,18 +260,24 @@ __global__ void read_slot_kernel(TrackState st, int seq, int slot, double* out72
     if (t < 64) out72[8 + t] = (double)c[t];
 }
 
-// One of a sequence's ordered slot lists as rows of LIST_COLS doubles: id, tlwh (from the Kalman mean, STrack.tlwh basetrack.py:183-211),
-// cls, score, slot, state, is_activated, tracklet_len, start_frame, frame_id.  out[cap * LIST_COLS] = the list length.
+// One of a sequence's ordered slot lists as rows of LIST_COLS doubles: id, tlwh (from the Kalman mean, STrack.tlwh basetrack.py:183-211;
+// C-BIoU: the last matched detection box), cls, score, slot, state, is_activated, tracklet_len, start_frame, frame_id.
+// out[cap * LIST_COLS] = the list length.
 constexpr int LIST_COLS = 13;
 template <class T>
-__global__ void read_list_kernel(TrackState st, int fmt, int seq, int which, double* out) {
+__global__ void read_list_kernel(TrackState st, int kind, int fmt, int seq, int which, double* out) {
     SeqView<T> v(st, seq);
     const int n = which == 0 ? v.ctrl[CTRL_NTRACKED] : v.ctrl[CTRL_NLOST];
     const int* list = which == 0 ? v.tracked : v.lost;
     for (int k = (int)threadIdx.x; k < n; k += (int)blockDim.x) {
         const int s = list[k];
         T box[4];
-        mean_to_tlwh<T>(fmt, v.mean + (size_t)s * 8, (v.flags[s] & 1) != 0, box);
+        if (kind == KIND_CBIOU) {
+            const T* h = v.cov + (size_t)s * 64 + CB_HIST + 4 * ((int)v.mean[(size_t)s * 8 + CB_LEN] - 1);
+            for (int q = 0; q < 4; ++q) box[q] = h[q];
+        } else {
+            mean_to_tlwh<T>(fmt, v.mean + (size_t)s * 8, (v.flags[s] & 1) != 0, box);
+        }
         double* o = out + (size_t)k * LIST_COLS;
         o[0] = (double)v.tid[s]; o[1] = (double)box[0]; o[2] = (double)box[1]; o[3] = (double)box[2]; o[4] = (double)box[3];
         o[5] = (double)v.cls[s]; o[6] = (double)v.score[s]; o[7] = (double)s; o[8] = (double)v.state[s]; o[9] = (double)v.activated[s];
@@ -446,11 +462,15 @@ static void layout(const b2t_tracker_config& c, unsigned char* base, b2t_tracker
 
 static int check_cfg(const b2t_tracker_config* c) {
     if (!c) return fail(B2T_EINVAL, "null config");
-    if (c->kind < 0 || c->kind > 2 || c->fmt < 0 || c->fmt > 2 || (c->dtype != B2T_F32 && c->dtype != B2T_F64))
+    if (c->kind < 0 || c->kind > 3 || (c->kind != B2T_CBIOU && (c->fmt < 0 || c->fmt > 2)) || (c->dtype != B2T_F32 && c->dtype != B2T_F64))
         return fail(B2T_EINVAL, "b2t_tracker: bad kind / fmt / dtype");
+    if (c->kind == B2T_CBIOU && c->dtype != B2T_F64)
+        return fail(B2T_EINVAL, "b2t_tracker: B2T_CBIOU runs in B2T_F64 only (the reference's buffered IoU is float64 and there is no Kalman "
+                                "state to shrink)");
     if (c->n_seq < 1 || c->cap < 64 || c->dmax < 1 || c->dmax > 1024 || c->cap > 4096 || c->ecap < 1)
         return fail(B2T_EINVAL, "b2t_tracker: bad n_seq / cap (64..4096) / dmax (1..1024) / ecap");
-    const size_t smem = c->dtype == B2T_F64 ? StepSmem<double>::bytes(c->cap, c->dmax, 0) : StepSmem<float>::bytes(c->cap, c->dmax, 0);
+    const size_t smem = c->kind == B2T_CBIOU ? cbiou_smem_bytes(c->cap, c->dmax, 0)
+                      : c->dtype == B2T_F64 ? StepSmem<double>::bytes(c->cap, c->dmax, 0) : StepSmem<float>::bytes(c->cap, c->dmax, 0);
     if (smem > 227 * 1024) return fail(B2T_ECAPACITY, "b2t_tracker: cap / dmax need more than 227 KB of shared memory per CTA");
     return B2T_OK;
 }
@@ -477,7 +497,9 @@ extern "C" int b2t_tracker_create(const b2t_tracker_config* cfg, void* state_mem
     size_t total;
     layout(*cfg, (unsigned char*)state_mem, t, &total);
     t->st.n_seq = cfg->n_seq; t->st.cap = cfg->cap; t->st.dmax = cfg->dmax; t->st.ecap = cfg->ecap;
-    t->st.esm = cfg->dtype == B2T_F64 ? StepSmem<double>::fit_esm(cfg->cap, cfg->dmax, cfg->ecap, 227 * 1024)
+    const bool cbiou = cfg->kind == B2T_CBIOU;
+    t->st.esm = cbiou ? cbiou_fit_esm(cfg->cap, cfg->dmax, cfg->ecap, 227 * 1024)
+              : cfg->dtype == B2T_F64 ? StepSmem<double>::fit_esm(cfg->cap, cfg->dmax, cfg->ecap, 227 * 1024)
                                       : StepSmem<float>::fit_esm(cfg->cap, cfg->dmax, cfg->ecap, 227 * 1024);
     t->out_rows_cap = cfg->cap;
     StepParams& p = t->prm;
@@ -488,10 +510,17 @@ extern "C" int b2t_tracker_create(const b2t_tracker_config* cfg, void* state_mem
     p.low_thresh = (float)((cfg->conf_thresh - 0.3) > 0.15 ? (cfg->conf_thresh - 0.3) : 0.15);  // bytetrack.py:15
     p.new_thresh = (float)(cfg->conf_thresh + 0.1);                                           // bytetrack.py:175
     if (cfg->kind == B2T_SORT) { p.t1 = cfg->iou_thresh; p.t2 = 0.0; p.t3 = cfg->iou_thresh + 0.1; }   // basetrack.py:414,438
-    else { p.t1 = 0.9; p.t2 = 0.5; p.t3 = 0.7; }                                              // bytetrack.py:118,137,160
+    else { p.t1 = 0.9; p.t2 = 0.5; p.t3 = 0.7; }                                              // bytetrack.py:118,137,160 ; c_biou_tracker.py:263,284,303
     p.t_dup = 0.15;                                                                           // basetrack.py:565
     p.max_time_lost = (int)(cfg->frame_rate / 30.0 * cfg->track_buffer);                      // basetrack.py:355-356
-    p.use_gmc = cfg->use_gmc; p.predict_only = 0;
+    p.use_gmc = cbiou ? 0 : cfg->use_gmc; p.predict_only = 0;
+    if (cbiou) {
+        t->smem = cbiou_smem_bytes(cfg->cap, cfg->dmax, t->st.esm);
+        auto k = cbiou_step_kernel<double>;
+        if (B2T_SET_SMEM(k, t->smem) != 0) { delete t; return fail(B2T_ECUDA, "cannot raise dynamic shared memory"); }
+        *out = t;
+        return b2t_tracker_reset(t, stream);
+    }
     t->smem = cfg->dtype == B2T_F64 ? StepSmem<double>::bytes(cfg->cap, cfg->dmax, t->st.esm) : StepSmem<float>::bytes(cfg->cap, cfg->dmax, t->st.esm);
     if (cfg->dtype == B2T_F64) { auto k = track_step_kernel<double>; if (B2T_SET_SMEM(k, t->smem) != 0) { delete t; return fail(B2T_ECUDA, "cannot raise dynamic shared memory"); } }
     else { auto k = track_step_kernel<float>; if (B2T_SET_SMEM(k, t->smem) != 0) { delete t; return fail(B2T_ECUDA, "cannot raise dynamic shared memory"); } }
@@ -507,10 +536,16 @@ extern "C" int b2t_tracker_step(b2t_tracker* t, const float* dets, const int* de
                                 const int* id_base, double* out, int out_rows, int* stat, int predict_only, void* stream) {
     if (!t || !out || !stat || out_rows < 1) return fail(B2T_EINVAL, "b2t_tracker_step: bad arguments");
     if (!predict_only && (!dets || !det_count)) return fail(B2T_EINVAL, "b2t_tracker_step: dets / det_count are NULL");
+    if (predict_only && t->cfg.kind == B2T_CBIOU)
+        return fail(B2T_EINVAL, "b2t_tracker_step: predict_only is not defined for B2T_CBIOU (the reference's update_without_detection "
+                                "predicts with a Kalman filter C-BIoU does not have)");
     StepParams p = t->prm;
     p.predict_only = predict_only ? 1 : 0;
     cudaStream_t s = (cudaStream_t)stream;
-    if (t->cfg.dtype == B2T_F64) {
+    if (t->cfg.kind == B2T_CBIOU) {
+        auto k = cbiou_step_kernel<double>;
+        B2T_LAUNCH(k, t->cfg.n_seq, 512, t->smem, s, t->st, p, dets, det_count, id_base, out, out_rows, stat);
+    } else if (t->cfg.dtype == B2T_F64) {
         auto k = track_step_kernel<double>;
         B2T_LAUNCH(k, t->cfg.n_seq, 512, t->smem, s, t->st, p, dets, det_count, warps, id_base, out, out_rows, stat);
     } else {
@@ -524,6 +559,9 @@ extern "C" int b2t_tracker_step_host(b2t_tracker* t, const float* dets_host, con
                                      const double* warps_host, const int* id_base_host, double* out_host, int out_rows,
                                      int* stat_host, int predict_only, void* stream) {
     if (!t || !out_host || !stat_host) return fail(B2T_EINVAL, "b2t_tracker_step_host: bad arguments");
+    if (predict_only && t->cfg.kind == B2T_CBIOU)
+        return fail(B2T_EINVAL, "b2t_tracker_step_host: predict_only is not defined for B2T_CBIOU (the reference's update_without_detection "
+                                "predicts with a Kalman filter C-BIoU does not have)");
     if (out_rows < 1 || (size_t)out_rows > t->out_rows_cap) return fail(B2T_EINVAL, "b2t_tracker_step_host: out_rows must be in [1, cap]");
     cudaStream_t s = (cudaStream_t)stream;
     const size_t S = t->cfg.n_seq;
@@ -551,8 +589,8 @@ extern "C" int b2t_tracker_read_list(b2t_tracker* t, int seq, int which, double*
     if (!t || seq < 0 || seq >= t->cfg.n_seq || (which != 0 && which != 1) || !rows_host || !n_host || max_rows < 0)
         return fail(B2T_EINVAL, "b2t_tracker_read_list: bad arguments");
     cudaStream_t s = (cudaStream_t)stream;
-    if (t->cfg.dtype == B2T_F64) { auto k = read_list_kernel<double>; B2T_LAUNCH(k, 1, 256, 0, s, t->st, t->cfg.fmt, seq, which, t->d_list); }
-    else { auto k = read_list_kernel<float>; B2T_LAUNCH(k, 1, 256, 0, s, t->st, t->cfg.fmt, seq, which, t->d_list); }
+    if (t->cfg.dtype == B2T_F64) { auto k = read_list_kernel<double>; B2T_LAUNCH(k, 1, 256, 0, s, t->st, t->cfg.kind, t->cfg.fmt, seq, which, t->d_list); }
+    else { auto k = read_list_kernel<float>; B2T_LAUNCH(k, 1, 256, 0, s, t->st, t->cfg.kind, t->cfg.fmt, seq, which, t->d_list); }
     int rc = check_launch("read_list");
     if (rc) return rc;
     double nd = 0;
